@@ -7,19 +7,17 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
-
-
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
 @pytest.fixture(scope="session")
-def reference_dir():
-    return REFERENCE if os.path.isdir(REFERENCE) else None
+def reference_strategy_dir():
+    """The original project's shipped strategy XML files, stored verbatim as test data."""
+    return os.path.join(ROOT, "tests", "golden", "reference_strategy")
 
 
-# The reference's 4-GPU sample strategy (same topology as /root/reference/strategy/4.xml), including
+# The reference's 4-GPU sample strategy (same topology as tests/golden/reference_strategy/4.xml), including
 # its malformed attribute list `id='1'ip='...'` (no separating space) that only tinyxml2 accepts.
 STRATEGY_4 = """<trees>
     <root id='0' ip='10.0.0.1'>

@@ -33,11 +33,9 @@ def test_xml_roundtrip_and_comments():
         xmlio.parse("<a><b></a")
 
 
-def test_all_reference_strategy_files_parse(reference_dir):
-    if reference_dir is None:
-        pytest.skip("reference tree not mounted")
-    files = sorted(glob.glob(os.path.join(reference_dir, "strategy", "*.xml")))
-    assert len(files) >= 10
+def test_all_reference_strategy_files_parse(reference_strategy_dir):
+    files = sorted(glob.glob(os.path.join(reference_strategy_dir, "*.xml")))
+    assert len(files) >= 16
     for f in files:
         s = Strategy.from_file(f, max_trees=64) if False else Strategy.from_xml(open(f).read(), max_trees=64)
         assert s.trees and all(t.root >= 0 for t in s.trees)
@@ -202,8 +200,8 @@ def test_python_and_native_parsers_agree_under_fuzzing():
     assert agree > 150
 
 
-def test_native_reader_accepts_every_shipped_and_reference_strategy_file(reference_dir):
-    """csrc/schedule.cpp against all strategy XML files of this repo and (when mounted) of the reference, including the
+def test_native_reader_accepts_every_shipped_and_reference_strategy_file(reference_strategy_dir):
+    """csrc/schedule.cpp against all strategy XML files of this repo and of the reference, including the
     reference's malformed-attribute dialect: same number of trees as the Python reader."""
     import glob
 
@@ -211,9 +209,8 @@ def test_native_reader_accepts_every_shipped_and_reference_strategy_file(referen
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     files = sorted(glob.glob(os.path.join(root, "strategy", "*.xml")))
-    if reference_dir:
-        files += sorted(glob.glob(os.path.join(reference_dir, "strategy", "*.xml")))
-    assert len(files) >= 10
+    files += sorted(glob.glob(os.path.join(reference_strategy_dir, "*.xml")))
+    assert len(files) >= 36
     for f in files:
         xml = open(f).read()
         s = Strategy.from_xml(xml)
